@@ -2,7 +2,7 @@
 """bench.py - speech-tokens/s of the GPT decode hot path (BASELINE.json metric), one JSON line.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference|torch-cuda]
-                    [--config c2|c3] [--path gpt|decoder]
+                    [--config c2|c3] [--path gpt|decoder] [--dump-outputs DIR]
 
 A "step" is one whole ``generate`` pass of the hot path over one batch: a 16-token prompt and
 ``--tokens`` (512) forced speech tokens per row, greedy + EOS excluded (BASELINE.json configs[1];
@@ -16,6 +16,8 @@ utterances sharded, one NCCL broadcast of the packed weights at load, no step-lo
 top-k 20 / penalty 1.05).  ``--path decoder``: hot path 2 at BASELINE configs[3] (DVAE decoder + Vocos + iSTFT of
 64 x 10 s), audio-samples/s with a tensor-core roofline against a TF32 peak measured in the same run.
 ``--impl torch-cuda``: the reference's own stack (HF LlamaModel, torch SDPA, eager PyTorch) on the same B200.
+``--dump-outputs DIR``: after the timed steps, what the timed path returned in its last step (rank 0) goes to
+``DIR/<name>.npy`` as float32; inputs are seeded, so two builds run with the same arguments can be compared file by file.
 """
 from __future__ import annotations
 
@@ -93,6 +95,22 @@ class ClockSampler:
         reasons = [n for i, n in enumerate(names) if any(len(r) > 3 + i and r[3 + i].lower().startswith("active") for r in self.rows)]
         return {"sm_mhz": sm[len(sm) // 2], "sm_max_mhz": int(self.rows[0][1]), "reasons": reasons,
                 "samples": len(sm)}
+
+
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Write each array as ``out_dir/<name>.npy`` in float32 (token ids are exact in float32: they are < 2**24)."""
+    import numpy as np
+
+    host = {name: a.detach().cpu().numpy().astype(np.float32) for name, a in arrays.items()}
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError(f"outputs of {total} B exceed the {DUMP_LIMIT_BYTES} B dump limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def build_inputs(B: int, tokens: int, seed: int):
@@ -176,6 +194,8 @@ def run_ours(args, rank: int, world: int, local_rank: int):
         ms = timed(step_resident, args.steps)
     launches = int(lib.ctb_launch_count() - l0)
     ms_per_step = ms / args.steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"ids": ids_out})  # [B, tokens, 4] speech-token ids of the last step
     value = world * B * tokens / (ms_per_step / 1e3)
 
     # ---- e2e through the public API with host buffers
@@ -415,9 +435,10 @@ def run_decoder(args, rank: int, world: int, local_rank: int):
     x_host = torch.randn(DEC_B, DEC_T, 768, generator=torch.Generator().manual_seed(1 + rank)).pin_memory()
     x_dev = x_host.to(dev)
     wav_host = torch.empty(DEC_B, 512 * DEC_T - 256, dtype=torch.float32).pin_memory()
+    last = {}
 
     def step_resident():
-        return dec.engine.tokens_to_wav(x_dev, 1)
+        last["wav"] = dec.engine.tokens_to_wav(x_dev, 1)
 
     def step_e2e():
         w = dec.engine.tokens_to_wav(x_host.to(dev, non_blocking=True), 1)
@@ -451,6 +472,9 @@ def run_decoder(args, rank: int, world: int, local_rank: int):
     with ClockSampler(local_rank) as clk:
         ms = timed(step_resident, args.steps) / args.steps
     launches = int(lib.ctb_launch_count() - l0)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"wav": last["wav"]})  # [64, 239872] waveforms, 61.4 MB
+    del last["wav"]
     samples = DEC_B * (512 * DEC_T - 256)
     value = world * samples / (ms / 1e3)
     step_e2e()
@@ -585,7 +609,7 @@ def run_torch_cuda(args, rank: int):
     for _ in range(max(1, min(args.warmup, 2))):
         gen(min(n, 32))
     torch.cuda.synchronize()
-    steps = max(1, min(args.steps, 3))
+    steps = args.steps
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(steps):
@@ -655,16 +679,18 @@ def run_c3(args, rank: int, world: int, local_rank: int):
     for _ in range(max(1, min(args.warmup, 2))):
         pipeline()
     barrier()
-    steps = max(1, min(args.steps, 3))
+    steps = args.steps
     l0 = lib.ctb_launch_count()
     with ClockSampler(local_rank) as clk:
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            pipeline()
+            code_ids = pipeline()
         e1.record()
         torch.cuda.synchronize()
         ms = e0.elapsed_time(e1) / steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"ids": torch.stack(code_ids)})  # [B, tokens, 4] code-pass ids of the last step
     if world > 1:
         t = torch.tensor([ms], device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -805,7 +831,13 @@ def main():
     ap.add_argument("--config", default="c2", choices=["c2", "c3"], help="c2: BASELINE configs[1] (default); c3: configs[2]")
     ap.add_argument("--path", default="gpt", choices=["gpt", "decoder"], help="decoder: hot path 2 at BASELINE configs[3]")
     ap.add_argument("--no-sweep", action="store_true", help="skip the short batch-8/32 and decoder side measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the timed path returned in "
+                    "its last step as DIR/<name>.npy (float32, seeded inputs: comparable between builds)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
 
     rank = int(os.environ.get("RANK", "0"))

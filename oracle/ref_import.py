@@ -1,9 +1,8 @@
 """Import the *unmodified* reference (``/root/reference``) inside the build container.
 
-TEST INFRASTRUCTURE ONLY.  Nothing under ``chattts_b200/`` may import this module; it is
-used by ``oracle/make_golden.py`` (fixture generation) and by the ``not gpu`` tests that
-pin ``oracle/*_oracle.py`` against the reference itself.  ``/root/reference`` does not
-exist on the GPU box, so nothing marked ``gpu`` may call :func:`load_reference`.
+TEST INFRASTRUCTURE ONLY.  Nothing under ``chattts_b200/`` may import this module; only
+``oracle/make_golden.py`` uses it, to write the fixtures under ``tests/golden/`` that the
+tests compare with, so no test needs the reference at run time.
 
 The reference cannot be imported as-is here (SURVEY.md §8c): ``vocos``,
 ``vector_quantize_pytorch`` and ``pybase16384`` are not installed and there is no network.

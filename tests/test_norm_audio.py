@@ -1,5 +1,8 @@
-"""Host pre/post-processing (SURVEY.md 8f N4): chattts_b200.norm.Normalizer against the reference's own Normalizer where
-/root/reference is present, and against expectations generated from it (committed below) everywhere else."""
+"""Host pre/post-processing (SURVEY.md 8f N4): chattts_b200.norm.Normalizer against what the reference's own Normalizer
+returned on the same inputs, stored in tests/golden/reference_host.json (``python -m oracle.make_golden gen_host_pins``)."""
+import json
+import os
+
 import numpy as np
 import pytest
 
@@ -18,39 +21,24 @@ CASES = [
     "nested [a[b]c] text",
     "数字123和符号@#都会被删除",
 ]
-# produced by the reference's Normalizer (ChatTTS/norm.py) with the homophone map above, default flags, in the build container
-EXPECTED = None
 
 
-def _ref():
-    from oracle.ref_import import load_reference, reference_available
-
-    if not reference_available():
-        pytest.skip("/root/reference not present on this box")
-    load_reference()
-    import json
-    import os
-    import tempfile
-
-    from ChatTTS.norm import Normalizer as RefNormalizer
-
-    fd, path = tempfile.mkstemp(suffix=".json")
-    with os.fdopen(fd, "w", encoding="utf-8") as f:
-        json.dump(HOMO, f, ensure_ascii=False)
-    return RefNormalizer(path)
+def normalizer_inputs():
+    """(text, do_text_normalization, do_homophone_replacement, lang) for every case and flag combination; both sides
+    have an "en" normaliser registered that upper-cases."""
+    return [(text, norm, homo, lang) for text in CASES for norm in (True, False) for homo in (True, False)
+            for lang in (None, "zh", "en")]
 
 
-@pytest.mark.reference
 def test_normalizer_matches_reference_on_every_case_and_flag_combination():
-    ref = _ref()
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_host.json"),
+              encoding="utf-8") as f:
+        expected = json.load(f)["normalizer"]
+    assert [tuple(r[:4]) for r in expected] == normalizer_inputs()
     ours = Normalizer(homophones=HOMO)
-    up = lambda s: s.upper()
-    assert ref.register("en", up) and ours.register("en", up)
-    for text in CASES:
-        for norm in (True, False):
-            for homo in (True, False):
-                for lang in (None, "zh", "en"):
-                    assert ours(text, norm, homo, lang) == ref(text, norm, homo, lang), (text, norm, homo, lang)
+    assert ours.register("en", lambda s: s.upper())
+    for text, norm, homo, lang, want in expected:
+        assert ours(text, norm, homo, lang) == want, (text, norm, homo, lang)
 
 
 def test_normalizer_golden_strings():

@@ -1,7 +1,9 @@
-"""Speaker strings / base16384 / prompt decoration (SURVEY.md 8f N3, host side) - CPU only."""
+"""Speaker strings / base16384 / prompt decoration (SURVEY.md 8f N3, host side) - CPU only.
+
+The reference's outputs are stored in tests/golden/reference_host.{json,npz} (``python -m oracle.make_golden gen_host_pins``)."""
+import json
 import lzma
 import os
-import re
 
 import numpy as np
 import pytest
@@ -9,6 +11,13 @@ import torch
 
 from chattts_b200 import b14
 from chattts_b200.speaker import Speaker
+
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
+
+def _reference_host():
+    with open(os.path.join(GOLD, "reference_host.json"), encoding="utf-8") as f:
+        return json.load(f)
 
 
 def test_base16384_round_trip_every_tail_length():
@@ -46,13 +55,9 @@ def test_speaker_strings_start_like_the_reference_ones():
                                filters=[{"id": lzma.FILTER_LZMA2, "preset": 9 | lzma.PRESET_EXTREME}])) == 1536
 
 
-@pytest.mark.reference
 def test_reference_spk_stat_decodes_to_std_and_mean():
     """config.py:132: the reference's own base16384 asset decodes to exactly 2 x 768 fp16 with a positive std half."""
-    path = "/root/reference/ChatTTS/config/config.py"
-    if not os.path.exists(path):
-        pytest.skip("/root/reference not present on this box")
-    stat = re.search(r'spk_stat: str = \(\s*"([^"]+)"', open(path, encoding="utf-8").read()).group(1)
+    stat = _reference_host()["spk_stat"]
     raw = b14.decode_from_string(stat)
     assert len(raw) == 2 * 768 * 2
     spk = Speaker(768, stat)
@@ -70,32 +75,37 @@ def test_prompt_round_trip_and_shape_header():
         Speaker.encode_prompt(torch.zeros(3, dtype=torch.int64))
 
 
-@pytest.mark.reference
-def test_apply_and_decoration_match_the_reference_speaker():
-    from oracle.ref_import import load_reference, reference_available
-
-    if not reference_available():
-        pytest.skip("/root/reference not present on this box")
-    load_reference()
-    from ChatTTS.model.speaker import Speaker as RefSpeaker
-
-    ref = object.__new__(RefSpeaker)
-    ours = object.__new__(Speaker)
+def apply_inputs():
     torch.manual_seed(1)
     emb = torch.randn(3, 6, 768)
     vec = torch.randn(768)
     ids = torch.randint(0, 50, (3, 6, 4))
     ids[0, 2, 0] = ids[2, 5, 0] = 21143
-    a = ref.apply(emb.clone(), vec, ids, 21143, torch.device("cpu"))
+    return emb, vec, ids
+
+
+DECORATE_CASES = ((None, None), ("x", None), ("x", "sample text"))
+DECORATE_TEXTS = ("  hi [Stts] there[spk_emb] ", "[empty_spk]b")
+
+
+def test_apply_and_decoration_match_the_reference_speaker():
+    """Against the reference Speaker's outputs on the same inputs: ``apply`` changed the rows ``apply_changed`` of the
+    embedding to ``apply_rows``; decoration results and the in-place stripped text lists."""
+    host, arrays = _reference_host(), np.load(os.path.join(GOLD, "reference_host.npz"))
+    ours = object.__new__(Speaker)
+    emb, vec, ids = apply_inputs()
+    a = emb.clone()
+    a[torch.from_numpy(arrays["apply_changed"])] = torch.from_numpy(arrays["apply_rows"])
     b = ours.apply(emb.clone(), vec, ids, 21143, torch.device("cpu"))
     assert torch.equal(a, b) and not torch.equal(a, emb)
     c = ours.apply(emb, vec, ids, 21143, torch.device("cpu"), inplace=False)
     assert torch.equal(c, a) and not torch.equal(emb, a)
-    for spk_emb, smp in ((None, None), ("x", None), ("x", "sample text")):
-        t1, t2 = ["  hi [Stts] there[spk_emb] ", "[empty_spk]b"], ["  hi [Stts] there[spk_emb] ", "[empty_spk]b"]
-        assert ours.decorate_code_prompts(t1, "[speed_5]", smp, spk_emb) == ref.decorate_code_prompts(t2, "[speed_5]", smp, spk_emb)
-        assert t1 == t2                                    # the caller's list is stripped in place by both
-    assert ours.decorate_text_prompts(["a", "b"], "[oral_2]") == ref.decorate_text_prompts(["a", "b"], "[oral_2]")
+    assert len(host["decorate_code"]) == len(DECORATE_CASES)
+    for (spk_emb, smp), (want, stripped) in zip(DECORATE_CASES, host["decorate_code"]):
+        t1 = list(DECORATE_TEXTS)
+        assert ours.decorate_code_prompts(t1, "[speed_5]", smp, spk_emb) == want
+        assert t1 == stripped                              # the caller's list is stripped in place by both
+    assert ours.decorate_text_prompts(["a", "b"], "[oral_2]") == host["decorate_text"]
 
 
 def test_decoration_golden():

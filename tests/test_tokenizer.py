@@ -1,7 +1,8 @@
 """chattts_b200.tokenizer.Tokenizer against the reference's Tokenizer on a small BERT vocabulary written on the fly."""
+import json
 import os
 
-import pytest
+import numpy as np
 import torch
 
 SPECIAL = ["[PAD]", "[UNK]", "[CLS]", "[SEP]", "[MASK]", "[Stts]", "[Ptts]", "[spk_emb]", "[empty_spk]", "[Sbreak]",
@@ -38,27 +39,26 @@ def test_layout_left_padding_and_audio_prompt(tmp_path):
     assert t.decode(ids[:, :, 0])[1].replace(" ", "").endswith("[Stts][empty_spk]hi[Ptts]")
 
 
-@pytest.mark.reference
+TEXTS = ("[Stts][spk_emb]hello there world[Ptts]", "[Stts][empty_spk]hi[Ptts]", "testing speech, a b.")
+PROMPT = torch.randint(0, 626, (4, 7), generator=torch.Generator().manual_seed(3))
+DECODE_IDS = [[16, 17, 11], [19, 12]]
+
+
 def test_matches_reference_tokenizer(tmp_path):
-    from oracle.ref_import import load_reference, reference_available
-
-    if not reference_available():
-        pytest.skip("/root/reference not present on this box")
-    load_reference()
-    from ChatTTS.model.tokenizer import Tokenizer as RefTokenizer
-
+    """Against the reference Tokenizer's outputs on the same vocabulary and inputs (tests/golden/reference_host.*,
+    ``python -m oracle.make_golden gen_host_pins``)."""
     from chattts_b200.tokenizer import Tokenizer
 
-    path = _write_vocab(tmp_path)
-    ours, ref = Tokenizer(path), RefTokenizer(path)
-    if not hasattr(ref._tokenizer, "encode_plus"):       # API drift: transformers >= 5 removed encode_plus (same as __call__)
-        ref._tokenizer.encode_plus = ref._tokenizer.__call__
-    assert (ours.len, ours.spk_emb_ids, ours.break_0_ids, ours.eos_token) == (ref.len, ref.spk_emb_ids, ref.break_0_ids, ref.eos_token)
-    texts = ["[Stts][spk_emb]hello there world[Ptts]", "[Stts][empty_spk]hi[Ptts]", "testing speech, a b."]
-    for prompt in (None, torch.randint(0, 626, (4, 7))):
-        a = ours.encode(list(texts), 4, prompt=prompt)
-        b = ref.encode(list(texts), 4, prompt=None if prompt is None else prompt.clone())
-        for x, y in zip(a, b):
-            assert x.dtype == y.dtype and torch.equal(x, y)
-    seq = [[16, 17, 11], [19, 12]]
-    assert ours.decode(seq) == ref.decode(seq)
+    gold = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+    with open(os.path.join(gold, "reference_host.json"), encoding="utf-8") as f:
+        ref = json.load(f)["tokenizer"]
+    arrays = np.load(os.path.join(gold, "reference_host.npz"))
+    ours = Tokenizer(_write_vocab(tmp_path))
+    assert (ours.len, ours.spk_emb_ids, ours.break_0_ids, ours.eos_token) == \
+        (ref["len"], ref["spk_emb_ids"], ref["break_0_ids"], ref["eos_token"])
+    for tag, prompt in (("noprompt", None), ("prompt", PROMPT)):
+        a = ours.encode(list(TEXTS), 4, prompt=prompt)
+        for x, name in zip(a, ("ids", "attention_mask", "text_mask")):
+            y = torch.from_numpy(arrays[f"tok_{tag}_{name}"])
+            assert x.dtype == y.dtype and torch.equal(x, y), (tag, name)
+    assert ours.decode(DECODE_IDS) == ref["decode"]

@@ -1,6 +1,6 @@
 import os, sys, torch
-sys.path.insert(0, "/root/repo")
-sys.path.insert(0, "/root/repo/tools")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 from flow_check import make, gen, time_steps
 ref, embed = make({"CTB_NO_FLOW": "1"})
 a, _ = make({"CTB_FLOW_NO_INK": "1"})
